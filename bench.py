@@ -41,6 +41,35 @@ def log(*a):
     print(*a, file=sys.stderr, flush=True)
 
 
+# ----------------------------------------------------------------------------- --dump-outputs
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SEED = 0
+_OUTPUTS = {}
+
+
+def keep_output(name, array):
+    "an array the timed path returned in its last step, saved as <name>.npy by write_outputs()"
+    array = np.ascontiguousarray(array)
+    assert array.dtype in (np.float32, np.float64), (name, array.dtype)
+    _OUTPUTS[name] = array
+
+
+def u64_as_float64(name, values):
+    "uint64 values as two exact float64 arrays (<name>_hi32, <name>_lo32): float64 holds 53 bits, a hash has 64"
+    values = np.asarray(values, dtype=np.uint64)
+    keep_output(name + "_hi32", (values >> np.uint64(32)).astype(np.float64))
+    keep_output(name + "_lo32", (values & np.uint64(0xFFFFFFFF)).astype(np.float64))
+
+
+def write_outputs(directory):
+    total = sum(a.nbytes for a in _OUTPUTS.values())
+    assert total <= DUMP_LIMIT_BYTES, "outputs to dump: %d bytes, more than %d" % (total, DUMP_LIMIT_BYTES)
+    os.makedirs(directory, exist_ok=True)
+    for name, array in sorted(_OUTPUTS.items()):
+        np.save(os.path.join(directory, name + ".npy"), array)
+    log(f"[bench] wrote {len(_OUTPUTS)} output arrays ({total} bytes) to {directory}")
+
+
 # stdout carries exactly one JSON line: keep a private handle to the real stdout and point fd 1
 # at stderr, so that library banners (e.g. "NCCL version ..." printed from C) cannot pollute it.
 _JSON_FD = None
@@ -368,6 +397,8 @@ def run_b200(args):
         if rank == 0:
             r.update({"n_gpus": world, "steps": args.steps, "warmup": args.warmup, "data": "synthetic", "dtype": "u64"})
             emit_json(r)
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs)
         if dist is not None:
             dist.destroy_process_group()
         return
@@ -382,6 +413,8 @@ def run_b200(args):
         if "compare" in out and "sketch" in out:
             line["sketch"] = out["sketch"]
         emit_json(line)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs)
     if dist is not None:
         dist.destroy_process_group()
 
@@ -410,6 +443,11 @@ def bench_compare(args, torch, dist, B, rank, world, timed, hbm_peak, peak_src):
 
         ms, launches, clocks, _ = timed(step_prof, args.steps, args.warmup)
         kernel_ms = kernel_ms[-args.steps:]
+        if args.dump_outputs:
+            # the whole 10000 x 10000 matrix is 800 MB: a fixed, seeded choice of whole rows of it
+            rows = np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=min(n, 256), replace=False))
+            keep_output("compare_jaccard_rows", d_out[torch.from_numpy(rows).to(dev)].cpu().numpy())
+            keep_output("compare_jaccard_row_ids", rows.astype(np.float64))
         # end to end: host CSR (pinned) -> H2D -> kernels -> D2H of the float64 matrix (pinned)
         ph, po = B.pinned_empty(len(h), np.uint64), B.pinned_empty(len(off), np.uint64)
         ph.array[:] = h
@@ -539,6 +577,11 @@ def bench_sketch(args, torch, dist, B, rank, world, timed, hbm_peak, peak_src):
 
     ms, launches, clocks, _ = timed(step, args.steps, args.warmup)
     kernel_ms = kernel_ms[-args.steps:]
+    if args.dump_outputs:
+        # one sketch per (genome, k), genome-major: ~1.5e6 hashes in all
+        hh, oo = last["sset"].to_host()
+        u64_as_float64("sketch_hashes", hh)
+        keep_output("sketch_offsets", np.asarray(oo, dtype=np.float64))
     pin = B.pinned_empty(len(my_seqs), np.uint8)
     pin.array[:] = my_seqs
 
@@ -748,6 +791,8 @@ def _bench_search(args, torch, dist, B, rank, world, timed, query, db, d_h, h_of
         def step_e2e():
             return int(sdb.search_counts(pq.array).sum())
     ms, launches, clocks, _ = timed(step, args.steps, args.warmup)
+    if args.dump_outputs:
+        keep_output("search_counts", d_counts[: hi - lo].cpu().numpy().astype(np.float64))
     ms_e2e, _, _, ex = timed(step_e2e, max(2, args.steps // 2), 1)
     alg = 8.0 * (n_hashes_total + nq * world)                    # every database hash once; the query once per rank
     achieved = alg / (ms / 1e3) / 1e9
@@ -830,6 +875,9 @@ def _bench_gather(args, torch, dist, B, rank, world, timed, query, db, d_h, h_of
             return len(ids)
     ms, launches, clocks, ex = timed(step, args.steps, args.warmup)
     ids, isizes = res["picks"]
+    if args.dump_outputs:
+        keep_output("gather_rows", np.asarray(ids, dtype=np.float64))
+        keep_output("gather_intersect_sizes", np.asarray(isizes, dtype=np.float64))
     out = {"metric": "gather wall time (configs[4])", "value": ms, "unit": "ms", "higher_is_better": False, "ms_per_step": ms,
            "scaling": "strong", "vs_baseline": None,
            "config": {"workload": GATHER_WORKLOAD, "query_hashes": int(len(query)), "db_rows": n_db, "parallelism": parallelism},
@@ -857,14 +905,23 @@ def _bench_gather(args, torch, dist, B, rank, world, timed, query, db, d_h, h_of
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5,
+                    help="timed steps of each workload; the end-to-end legs (host buffers in and out) run "
+                         "max(2, steps // 2) more")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default=None, choices=["compare", "sketch", "both", "search", "gather"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--index", action="store_true",
                     help="search / gather workloads: query through the inverted index of the resident database")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, save what the last timed step computed as DIR/<name>.npy "
+                         "(float32/float64, at most 64 MB, a fixed seeded sample of larger outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or int(os.environ.get("WORLD_SIZE", "1")) != 1):
+        ap.error("--dump-outputs needs --impl b200 in a single process")
     if args.workload is None:
         args.workload = "compare" if args.impl == "reference" else "both"
     if args.warmup < 3 and args.impl == "b200":

@@ -71,6 +71,17 @@ def s10_records():
 
 
 @pytest.fixture(scope="session")
+def reference_corpus(tmp_path_factory):
+    """golden/reference_corpus.tar.gz extracted: sourmash's test data, shrunk (golden/make_reference_corpus.py), laid out
+    as in a sourmash checkout (tests/test-data/, data/).  Returns the directory."""
+    import tarfile
+    root = tmp_path_factory.mktemp("reference_corpus")
+    with tarfile.open(os.path.join(GOLDEN, "reference_corpus.tar.gz")) as tar:
+        tar.extractall(root, filter="data")
+    return str(root)
+
+
+@pytest.fixture(scope="session")
 def golden_dir():
     import pathlib
     return pathlib.Path(GOLDEN)

@@ -99,12 +99,13 @@ LINES = []
 bench.emit_json = lambda obj: LINES.append(json.loads(json.dumps(obj)))
 
 
-def run(workload, env=None, extra=(), cpu_baseline=False):
+def run(workload, env=None, extra=(), cpu_baseline=False, dump_outputs=None):
     old = {k: os.environ.get(k) for k in (env or {})}
     os.environ.update(env or {})
     try:
         args = types.SimpleNamespace(gpus=1, steps=1, warmup=3, impl="b200", workload=workload, no_cpu_baseline=not cpu_baseline,
-                                     index="--index" in extra)
+                                     index="--index" in extra, dump_outputs=dump_outputs)
+        bench._OUTPUTS.clear()
         n0 = len(LINES)
         bench.run_b200(args)
         assert len(LINES) == n0 + 1, "one JSON line per run"
@@ -150,6 +151,28 @@ def main():
         assert "index" in indexed and indexed["index"]["distinct_hashes"] > 0 and "index" not in plain
         if workload == "gather":
             assert plain["rounds"] == ranged["rounds"] == indexed["rounds"] > 2, (plain["rounds"], ranged["rounds"], indexed["rounds"])
+    # --dump-outputs: what the last timed step returned, float64 files, the same on a second run with the same arguments
+    import tempfile
+    with tempfile.TemporaryDirectory() as tmp:
+        for workload, names in (("both", {"compare_jaccard_rows", "compare_jaccard_row_ids", "sketch_hashes_hi32",
+                                          "sketch_hashes_lo32", "sketch_offsets"}),
+                                ("search", {"search_counts"}), ("gather", {"gather_rows", "gather_intersect_sizes"})):
+            first, second = os.path.join(tmp, workload + "1"), os.path.join(tmp, workload + "2")
+            run(workload, dump_outputs=first)
+            run(workload, dump_outputs=second)
+            assert set(os.listdir(first)) == {n + ".npy" for n in names}, sorted(os.listdir(first))
+            for f in os.listdir(first):
+                a, b = np.load(os.path.join(first, f)), np.load(os.path.join(second, f))
+                assert a.dtype == np.float64 and a.size and np.array_equal(a, b), f
+        rows = np.load(os.path.join(tmp, "both1", "compare_jaccard_rows.npy"))
+        ids = np.load(os.path.join(tmp, "both1", "compare_jaccard_row_ids.npy")).astype(np.int64)
+        assert rows.shape == (len(ids), len(_small_compare()[1]) - 1) and np.array_equal(rows[:, ids], rows[:, ids].T)
+        hi, lo = (np.load(os.path.join(tmp, "both1", "sketch_hashes_%s32.npy" % p)).astype(np.uint64) for p in ("hi", "lo"))
+        off = np.load(os.path.join(tmp, "both1", "sketch_offsets.npy")).astype(np.int64)
+        hashes = (hi << np.uint64(32)) | lo
+        assert len(off) == bench.N_GENOMES * len(bench.KSIZES) + 1 and off[-1] == len(hashes)
+        from sourmash_b200.synth import MAX_HASH_1000
+        assert len(hashes) and (hashes <= np.uint64(MAX_HASH_1000)).all()   # exact: the split keeps all 64 bits
     print("bench dry run ok: %d JSON lines assembled" % len(LINES))
 
 

@@ -177,17 +177,19 @@ def test_gather_fixture_bruteforce_matches_reference_expectation(golden):
     assert got == golden["meta"]["gather_k21_expected"]
 
 
-REF_DATA = "/root/reference/tests/test-data"
+@pytest.fixture(scope="module")
+def ref_data(reference_corpus):
+    "sourmash's test-data directory (shrunk; see the reference_corpus fixture)"
+    return os.path.join(reference_corpus, "tests", "test-data")
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="reference checkout not present (build container only)")
-def test_native_parser_on_the_reference_fixture_corpus():
+def test_native_parser_on_the_reference_fixture_corpus(ref_data):
     """Every .sig / .sig.gz the reference ships as test data (hundreds of files: old writers,
     abundances, protein / dayhoff / hp, num and scaled, multi-signature files) through the native
     parser, against Python's json on the same bytes."""
     import glob
-    paths = sorted(glob.glob(os.path.join(REF_DATA, "**", "*.sig"), recursive=True) +
-                   glob.glob(os.path.join(REF_DATA, "**", "*.sig.gz"), recursive=True))
+    paths = sorted(glob.glob(os.path.join(ref_data, "**", "*.sig"), recursive=True) +
+                   glob.glob(os.path.join(ref_data, "**", "*.sig.gz"), recursive=True))
     assert len(paths) > 100
     checked = sketches = 0
     for p in paths:
@@ -242,13 +244,12 @@ def _py_records(path):
     return out
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="reference checkout not present (build container only)")
-def test_native_reader_on_the_reference_sequence_files():
+def test_native_reader_on_the_reference_sequence_files(ref_data):
     import glob
     paths = []
     for pat in ("*.fa", "*.fa.gz", "*.fna", "*.fna.gz", "*.faa", "*.faa.gz", "*.fq.gz", "*.fq", "*.fastq", "*.fasta"):
-        paths += glob.glob(os.path.join(REF_DATA, "**", pat), recursive=True)
-        paths += glob.glob(os.path.join(os.path.dirname(os.path.dirname(REF_DATA)), "data", pat))
+        paths += glob.glob(os.path.join(ref_data, "**", pat), recursive=True)
+        paths += glob.glob(os.path.join(os.path.dirname(os.path.dirname(ref_data)), "data", pat))
     paths = sorted(set(p for p in paths if os.path.getsize(p) > 0))
     assert len(paths) > 12
     checked = 0

@@ -1,21 +1,32 @@
-"""`sourmash scripts b200sketch | b200compare | b200search | b200gather | b200prefetch` through the REFERENCE's command line.
+"""`sourmash scripts b200sketch | b200compare | b200search | b200gather | b200prefetch` against the REFERENCE's own commands.
 
 north_star asks for the hot paths "behind the reference's own plugin API": the reference loads command plugins from the
-entry-point group `sourmash.cli_script` (src/sourmash/plugins.py:8-12, 91-186).  Here the reference's package (loaded in
-place over this library, as in test_reference_python_over_abi.py) finds this package's entry points in a dist-info written
-next to it, and every plugin command is run next to the reference's own command on the same inputs:
+entry-point group `sourmash.cli_script` (src/sourmash/plugins.py:8-12, 91-186).  Every plugin command is compared with the
+reference's own command on the same inputs:
 
     sourmash sketch dna / protein / translate   vs   sourmash scripts b200sketch      -> equal signatures
     sourmash compare                            vs   sourmash scripts b200compare     -> equal matrix, labels, CSV
     sourmash search / gather / prefetch         vs   sourmash scripts b200search ...  -> byte-identical CSV files
 
-Both sides run on the emulated library (no GPU where the reference checkout is); the reference's commands go sketch by
-sketch and pair by pair through the C ABI, the plugin commands through this package's batched entry points."""
+The reference's outputs are stored in golden/plugin_cli.tar.gz; the plugin commands run here (`python -m
+sourmash_b200.plugin`, on the emulated library, so no GPU is needed).  The inputs are the sourmash test data the suite
+stores: golden/reference_corpus.tar.gz with the full-size files of golden/ laid over it.  With SOURMASH_CHECKOUT naming a
+sourmash checkout, the reference's commands run live instead (its package loaded in place over the emulated library, as in
+test_reference_python_over_abi.py, and finding this package's entry points in a dist-info written next to it) and the
+archive is written anew from what they produce."""
 import csv
 import glob
+import gzip
+import io
+import json
 import os
+import shutil
 import subprocess
 import sys
+import tarfile
+import zipfile
+import zlib
+from types import SimpleNamespace
 
 import numpy as np
 import pytest
@@ -23,60 +34,126 @@ import pytest
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 import test_reference_python_over_abi as over_abi  # noqa: E402
 
-REF = over_abi.REF
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-DATA = os.path.join(REF, "tests", "test-data")
-
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "src", "sourmash")),
-                                reason="needs the reference checkout (this container only)")
+GOLDEN = os.path.join(HERE, "golden")
+STORED = os.path.join(GOLDEN, "plugin_cli.tar.gz")
+CHECKOUT = os.environ.get("SOURMASH_CHECKOUT")
+DATA = "data"                   # the inputs, relative to the working directory: the reports quote these paths
+WORK_MARK = "{WORK}"            # the absolute working directory in stored text (a zip database reports its absolute path)
+FULL_SIZE = ["gather", "47.fa.sig", "63.fa.sig", "2.fa.sig", "genome-s10.fa.gz", "ecoli.faa", "ecoli.genes.fna"]
 
 COMMANDS = ("B200Sketch", "B200Compare", "B200Search", "B200Gather", "B200Prefetch")
 
 
+def _outputs(args):
+    "the files a reference command line writes: -o, --csv, and the labels next to a compare matrix"
+    out = [args[i + 1] for i, a in enumerate(args[:-1]) if a in ("-o", "--csv")]
+    return out + [o + ".labels.txt" for o in out if o.endswith(".npy")]
+
+
+def cat_signatures(paths, out):
+    "the signatures of `paths` in one .sig file, or in one .zip with a manifest and one signatures/<md5>.sig.gz per sketch, as `sig cat` writes them"
+    records = []
+    for p in paths:
+        with open(p) as fh:
+            records += json.load(fh)
+    if not out.endswith(".zip"):
+        with open(out, "w") as fh:
+            json.dump(records, fh)
+        return
+    rows = ["# SOURMASH-MANIFEST-VERSION: 1.0\n"
+            "internal_location,md5,md5short,ksize,moltype,num,scaled,n_hashes,with_abundance,name,filename\n"]
+    with zipfile.ZipFile(out, "w") as z:
+        for rec, sk in ((r, sk) for r in records for sk in r["signatures"]):      # one member and one row per sketch
+            member = "signatures/%s.sig.gz" % sk["md5sum"]
+            z.writestr(member, gzip.compress(json.dumps([dict(rec, signatures=[sk])]).encode(), mtime=0))
+            scaled = (2**64 - 1) // sk["max_hash"] if sk.get("max_hash") else 0      # what sourmash derives from max_hash
+            rows.append(",".join([member, sk["md5sum"], sk["md5sum"][:8], str(sk["ksize"]), sk.get("molecule", "dna").upper(),
+                                  str(0 if scaled else sk.get("num", 0)), str(scaled), str(len(sk["mins"])), str(int("abundances" in sk)),
+                                  '"%s"' % (rec.get("name") or ""), '"%s"' % (rec.get("filename") or "")]) + "\n")
+        z.writestr("SOURMASH-MANIFEST.csv", "".join(rows))
+
+
 @pytest.fixture(scope="module")
-def cli(tmp_path_factory):
+def cli(tmp_path_factory, reference_corpus):
     sys.path.insert(0, os.path.join(HERE, "host_emul"))
     try:
         import emul_lib
     finally:
         sys.path.pop(0)
     tmp = str(tmp_path_factory.mktemp("refcli"))
-    over_abi._stub_package(tmp, emul_lib.build())
     site = os.path.join(tmp, "site")
-    info = os.path.join(site, "sourmash_b200-0.1.0.dist-info")         # what `pip install .` writes from pyproject.toml
-    os.makedirs(info)
-    with open(os.path.join(info, "METADATA"), "w") as fh:
-        fh.write("Metadata-Version: 2.1\nName: sourmash_b200\nVersion: 0.1.0\n")
+    os.makedirs(site)
+    env = dict(os.environ, PYTHONPATH=site, PYTHONDONTWRITEBYTECODE="1")
+    if CHECKOUT:
+        over_abi.REF = CHECKOUT
+        over_abi._stub_package(tmp, emul_lib.build())
+        info = os.path.join(site, "sourmash_b200-0.1.0.dist-info")     # what `pip install .` writes from pyproject.toml
+        os.makedirs(info)
+        with open(os.path.join(info, "METADATA"), "w") as fh:
+            fh.write("Metadata-Version: 2.1\nName: sourmash_b200\nVersion: 0.1.0\n")
+        with open(os.path.join(info, "entry_points.txt"), "w") as fh:
+            fh.write("[sourmash.cli_script]\n" + "".join("%s = sourmash_b200.plugin:Command_%s\n" % (c.lower(), c) for c in COMMANDS))
+        env["PYTHONPATH"] = os.pathsep.join([site, os.path.join(tmp, "reftests")])
     with open(os.path.join(ROOT, "pyproject.toml")) as fh:
         declared = [line.split("=")[0].strip() for line in fh if "sourmash_b200.plugin:Command_" in line]
-    assert declared == [c.lower() for c in COMMANDS]                   # the entry points written below are the declared ones
-    with open(os.path.join(info, "entry_points.txt"), "w") as fh:
-        fh.write("[sourmash.cli_script]\n" + "".join("%s = sourmash_b200.plugin:Command_%s\n" % (c.lower(), c) for c in COMMANDS))
-    with open(os.path.join(site, "sitecustomize.py"), "w") as fh:       # this package too binds the emulated library
+    assert declared == [c.lower() for c in COMMANDS]                   # the entry points are the declared ones
+    with open(os.path.join(site, "sitecustomize.py"), "w") as fh:       # this package binds the emulated library
         fh.write("import sys\nsys.path.insert(0, %r); sys.path.insert(0, %r)\nimport emulated_boot\nemulated_boot.install()\n"
                  % (os.path.join(HERE, "host_emul"), ROOT))
-    env = dict(os.environ, PYTHONPATH=os.pathsep.join([site, os.path.join(tmp, "reftests")]), PYTHONDONTWRITEBYTECODE="1")
     work = os.path.join(tmp, "work")
-    os.makedirs(work)
+    shutil.copytree(os.path.join(reference_corpus, "tests", "test-data"), os.path.join(work, DATA))
+    for name in FULL_SIZE:                                               # full-size copies of the files golden/ holds
+        src = os.path.join(GOLDEN, name)
+        if os.path.isdir(src):
+            shutil.copytree(src, os.path.join(work, DATA, name), dirs_exist_ok=True)
+        else:
+            shutil.copy(src, os.path.join(work, DATA, name))
+    stored = {}
+    if not CHECKOUT:
+        with tarfile.open(STORED) as tar:
+            stored = {m.name: tar.extractfile(m).read() for m in tar.getmembers()}
+
+    def _text(data, to_stored):
+        a, b = (work.encode(), WORK_MARK.encode()) if to_stored else (WORK_MARK.encode(), work.encode())
+        return data.replace(a, b)
 
     def run(*args, rc=(0,)):
-        r = subprocess.run([sys.executable, "-m", "sourmash"] + [str(a) for a in args], capture_output=True, text=True, env=env,
-                           cwd=work, timeout=900)
-        assert r.returncode in rc, " ".join(map(str, args)) + "\n" + r.stdout[-2000:] + r.stderr[-3000:]
-        return r
+        args = [str(a) for a in args]
+        if args[0] == "scripts" and len(args) > 1 and args[1].startswith("b200"):   # the plugin: this package, here
+            r = subprocess.run([sys.executable, "-m", "sourmash_b200.plugin"] + args[1:], capture_output=True, text=True,
+                               env=env, cwd=work, timeout=900)
+            assert r.returncode in rc, " ".join(args) + "\n" + r.stdout[-2000:] + r.stderr[-3000:]
+            return r
+        key = " ".join(args)                                             # the reference: stored outputs, or run live
+        if CHECKOUT:
+            r = subprocess.run([sys.executable, "-m", "sourmash"] + args, capture_output=True, text=True, env=env,
+                               cwd=work, timeout=900)
+            assert r.returncode in rc, key + "\n" + r.stdout[-2000:] + r.stderr[-3000:]
+            stored["console/" + key.replace("/", "|")] = _text((r.stdout + r.stderr).encode(), True)
+            for name in _outputs(args):
+                with open(os.path.join(work, name), "rb") as fh:
+                    stored[name] = _text(fh.read(), True)
+            return r
+        for name in _outputs(args):
+            assert name in stored, "no stored reference output for: " + key
+            with open(os.path.join(work, name), "wb") as fh:
+                fh.write(_text(stored[name], False))
+        out = _text(stored.get("console/" + key.replace("/", "|"), b""), False).decode()
+        return SimpleNamespace(returncode=0, stdout=out, stderr="")
 
-    def load(path):                                                      # with the reference's own loader
-        code = ("import sourmash, sys, json\n"
+    def load(path):                                                      # this package's loader
+        code = ("import sourmash_b200 as s, sys, json\n"
                 "print(json.dumps(sorted([ss.name, ss.filename, ss.md5sum(), ss.minhash.ksize, ss.minhash.moltype, "
                 "ss.minhash.scaled, ss.minhash.num, int(ss.minhash.track_abundance), sorted(ss.minhash.hashes.items())] "
-                "for ss in sourmash.load_file_as_signatures(sys.argv[1]))))")
+                "for ss in s.load_file_as_signatures(sys.argv[1]))))")
         r = subprocess.run([sys.executable, "-c", code, path], capture_output=True, text=True, env=env, cwd=work, timeout=900)
         assert r.returncode == 0, r.stderr[-3000:]
         return r.stdout
 
     def together(*cmdlines):
-        "several command lines at once (each is a process that spends a second importing the reference package)"
+        "several command lines at once (each is a process that spends a second importing its package)"
         from concurrent.futures import ThreadPoolExecutor
         with ThreadPoolExecutor(len(cmdlines)) as pool:
             return list(pool.map(lambda c: run(*c), cmdlines))
@@ -87,14 +164,26 @@ def cli(tmp_path_factory):
             return list(pool.map(load, paths))
 
     run.work, run.load, run.loads, run.together = work, load, loads, together
-    return run
+    run.glob = lambda pattern: [os.path.relpath(p, work) for p in glob.glob(os.path.join(work, pattern))]
+    yield run
+    if CHECKOUT:                                                         # the reference's outputs, for runs without it
+        buf = io.BytesIO()
+        with tarfile.open(fileobj=buf, mode="w") as tar:
+            for name in sorted(stored):
+                ti = tarfile.TarInfo(name)
+                ti.size, ti.mode = len(stored[name]), 0o644
+                tar.addfile(ti, io.BytesIO(stored[name]))
+        with open(STORED, "wb") as fh:
+            fh.write(gzip.compress(buf.getvalue(), compresslevel=9, mtime=0))
 
 
 def test_the_reference_lists_the_plugin_commands(cli):
     r = cli("scripts", rc=(0, 1))                          # no command given: the list of commands, exit status 1
     out = r.stderr + r.stdout
+    from sourmash_b200 import plugin
     for c in COMMANDS:
         assert "sourmash scripts %s" % c.lower() in out
+        assert getattr(plugin, "Command_" + c).description in out
 
 
 @pytest.mark.parametrize("kind,params,files", [
@@ -106,7 +195,7 @@ def test_the_reference_lists_the_plugin_commands(cli):
 ])
 def test_sketch_commands_write_equal_signatures(cli, kind, params, files):
     paths = [os.path.join(DATA, f) for f in files]
-    tag = "%s_%s" % (kind, abs(hash(params)) % 10**6)
+    tag = "%s_%08x" % (kind, zlib.crc32(params.encode()))
     extra, plugin_params = [], params
     if kind != "dna":
         moltype = "dayhoff" if "dayhoff" in params else "hp" if ",hp" in params else "protein"
@@ -150,7 +239,7 @@ def test_sketch_of_fastq_and_invalid_bases(cli):
 
 
 def test_compare_command_writes_the_same_matrix(cli):
-    sigs = sorted(glob.glob(os.path.join(DATA, "gather", "GCF*.sig")))
+    sigs = sorted(cli.glob(os.path.join(DATA, "gather", "GCF*.sig")))
     cli.together(["compare", *sigs, "-k", "21", "-o", "ref.npy", "--csv", "ref_cmp.csv"],
                  ["scripts", "b200compare", *sigs, "-k", "21", "-o", "b200.npy", "--csv", "b200_cmp.csv"])
     w = cli.work
@@ -165,7 +254,7 @@ def test_compare_command_writes_the_same_matrix(cli):
                                    ["--distance-matrix"], ["--scaled", "2000"]])
 def test_compare_flags_write_the_same_matrix(cli, flags):
     "the other matrices of `sourmash compare`: containment forms, ANI, distances, a coarser --scaled"
-    sigs = sorted(glob.glob(os.path.join(DATA, "gather", "GCF*.sig")))[:6]
+    sigs = sorted(cli.glob(os.path.join(DATA, "gather", "GCF*.sig")))[:6]
     tag = "cmp" + "".join(flags).replace("-", "")
     cli.together(["compare", *sigs, "-k", "21", "-o", tag + "_ref.npy", "--csv", tag + "_ref.csv", *flags],
                  ["scripts", "b200compare", *sigs, "-k", "21", "-o", tag + "_b200.npy", "--csv", tag + "_b200.csv", *flags])
@@ -193,7 +282,7 @@ def _same_file(cli, a, b, min_rows):
 
 @pytest.mark.parametrize("flags", [[], ["--containment"], ["--max-containment"], ["--best-only"]])
 def test_search_command_writes_the_same_csv(cli, flags):
-    sigs = sorted(glob.glob(os.path.join(DATA, "gather", "GCF*.sig")))
+    sigs = sorted(cli.glob(os.path.join(DATA, "gather", "GCF*.sig")))
     tag = "search" + "".join(flags).replace("-", "")
     cli.together(["search", sigs[0], *sigs, "-k", "21", "--threshold", "0.01", "-o", tag + "_ref.csv", *flags],
                  ["scripts", "b200search", sigs[0], *sigs, "-k", "21", "--threshold", "0.01", "-o", tag + "_b200.csv", *flags])
@@ -203,7 +292,7 @@ def test_search_command_writes_the_same_csv(cli, flags):
 @pytest.mark.parametrize("threshold_bp", ["0", "50000"])
 def test_gather_and_prefetch_commands_write_the_same_csv(cli, threshold_bp):
     query = os.path.join(DATA, "gather", "combined.sig")
-    sigs = sorted(glob.glob(os.path.join(DATA, "gather", "GCF*.sig")))
+    sigs = sorted(cli.glob(os.path.join(DATA, "gather", "GCF*.sig")))
     for cmd in ("gather", "prefetch"):
         tag = "%s_%s" % (cmd, threshold_bp)
         cli.together([cmd, query, *sigs, "-k", "21", "--threshold-bp", threshold_bp, "-o", tag + "_ref.csv"],
@@ -222,10 +311,10 @@ def test_gather_of_an_abundance_query_writes_the_same_csv(cli):
 
 @pytest.mark.parametrize("flags", [[], ["--best-only"], ["--containment", "--best-only"]])
 def test_search_of_one_multi_signature_database(cli, flags):
-    "all subjects in ONE file (made with the reference's `sig cat`): --best-only ratchets its threshold inside a database"
-    sigs = sorted(glob.glob(os.path.join(DATA, "gather", "GCF*.sig")))
+    "all subjects in ONE file: --best-only ratchets its threshold inside a database"
+    sigs = sorted(cli.glob(os.path.join(DATA, "gather", "GCF*.sig")))
     if not os.path.exists(os.path.join(cli.work, "all12.sig")):
-        cli("sig", "cat", *sigs[::-1], "-o", "all12.sig")              # reversed: the query's own sketch comes last
+        cat_signatures([os.path.join(cli.work, p) for p in sigs[::-1]], os.path.join(cli.work, "all12.sig"))   # query's own last
     tag = "one" + "".join(flags).replace("-", "")
     cli.together(["search", sigs[3], "all12.sig", "-k", "21", "--threshold", "0.01", "-o", tag + "_ref.csv", *flags],
                  ["scripts", "b200search", sigs[3], "all12.sig", "-k", "21", "--threshold", "0.01", "-o", tag + "_b200.csv", *flags])
@@ -236,10 +325,10 @@ def test_search_of_one_multi_signature_database(cli, flags):
 
 
 def test_a_zip_collection_as_the_database(cli):
-    "the twelve genomes in one .zip (written by the reference's `sig cat`): every command, same files; a zip reports its absolute path"
-    sigs = sorted(glob.glob(os.path.join(DATA, "gather", "GCF*.sig")))
+    "the twelve genomes in one .zip: every command, same files; a zip reports its absolute path"
+    sigs = sorted(cli.glob(os.path.join(DATA, "gather", "GCF*.sig")))
     query = os.path.join(DATA, "gather", "combined.sig")
-    cli("sig", "cat", *sigs, "-o", "all12.zip")
+    cat_signatures([os.path.join(cli.work, p) for p in sigs], os.path.join(cli.work, "all12.zip"))
     cli.together(["gather", query, "all12.zip", "-k", "21", "--threshold-bp", "0", "-o", "zip_gather_ref.csv"],
                  ["scripts", "b200gather", query, "all12.zip", "-k", "21", "--threshold-bp", "0", "-o", "zip_gather_b200.csv"],
                  ["prefetch", query, "all12.zip", "-k", "21", "--threshold-bp", "0", "-o", "zip_prefetch_ref.csv"],
@@ -258,12 +347,12 @@ def test_a_directory_as_the_database_and_the_scaled_option(cli):
     """A directory (with a sub-directory) of .sig files is one database whose matches report the file they came from; --scaled
     downsamples the query first, and the reports then quote that sketch; protein sketches."""
     import shutil
-    sigs = sorted(glob.glob(os.path.join(DATA, "gather", "GCF*.sig")))
+    sigs = sorted(cli.glob(os.path.join(DATA, "gather", "GCF*.sig")))
     query = os.path.join(DATA, "gather", "combined.sig")
     db = os.path.join(cli.work, "dbdir")
     os.makedirs(os.path.join(db, "sub"))
     for i, p in enumerate(sigs):
-        shutil.copy(p, os.path.join(db, "sub") if i % 3 == 0 else db)
+        shutil.copy(os.path.join(cli.work, p), os.path.join(db, "sub") if i % 3 == 0 else db)
     cli.together(["gather", query, "dbdir", "-k", "21", "--threshold-bp", "0", "-o", "dir_gather_ref.csv"],
                  ["scripts", "b200gather", query, "dbdir", "-k", "21", "--threshold-bp", "0", "-o", "dir_gather_b200.csv"],
                  ["search", sigs[0], "dbdir", "--best-only", "-k", "21", "--threshold", "0.01", "-o", "dir_search_ref.csv"],
@@ -276,7 +365,7 @@ def test_a_directory_as_the_database_and_the_scaled_option(cli):
     _same_file(cli, "dir_search_ref.csv", "dir_search_b200.csv", 1)
     _same_file(cli, "sc_gather_ref.csv", "sc_gather_b200.csv", 3)
     assert np.array_equal(np.load(os.path.join(cli.work, "dir_ref.npy")), np.load(os.path.join(cli.work, "dir_b200.npy")))
-    prot = sorted(glob.glob(os.path.join(DATA, "prot", "protein", "*.sig")))
+    prot = sorted(cli.glob(os.path.join(DATA, "prot", "protein", "*.sig")))
     cli.together(["search", prot[0], *prot, "--protein", "--threshold", "0.0", "-o", "prot_search_ref.csv"],
                  ["scripts", "b200search", prot[0], *prot, "--moltype", "protein", "--threshold", "0.0", "-o", "prot_search_b200.csv"],
                  ["gather", prot[0], *prot, "--protein", "--threshold-bp", "0", "-o", "prot_gather_ref.csv"],
@@ -288,7 +377,7 @@ def test_a_directory_as_the_database_and_the_scaled_option(cli):
 def test_confidence_interval_columns(cli):
     "--estimate-ani-ci: the four (gather, prefetch) / two (containment search) extra columns"
     query = os.path.join(DATA, "gather", "combined.sig")
-    sigs = sorted(glob.glob(os.path.join(DATA, "gather", "GCF*.sig")))
+    sigs = sorted(cli.glob(os.path.join(DATA, "gather", "GCF*.sig")))
     pairs = []
     for cmd, first, flags in (("gather", query, ["--threshold-bp", "0"]), ("prefetch", query, ["--threshold-bp", "0"]),
                               ("search", sigs[0], ["--threshold", "0.01", "--containment"])):

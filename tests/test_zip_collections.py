@@ -24,9 +24,6 @@ from sourmash_b200.sigset import SignatureSet
 from tests.conftest import GOLDEN
 from tests.test_index_glue import _FakeSet, cpu_kernels  # noqa: F401  (fixture)
 
-REF_DATA = "/root/reference/tests/test-data"
-needs_reference = pytest.mark.skipif(not os.path.isdir(REF_DATA),
-                                     reason="reference checkout not present (build container only)")
 GATHER = sorted(glob.glob(os.path.join(GOLDEN, "gather", "GCF*.sig")))
 
 
@@ -342,12 +339,17 @@ def test_zipfile_search_matches_linear_index(zip_db, cpu_kernels, monkeypatch):
 
 
 # ---------------------------------------------------------------------------------------------
-# the reference's own archives (build container only)
+# the reference's own archives, shrunk (golden/make_reference_corpus.py: every member kept, sketches cut short)
 # ---------------------------------------------------------------------------------------------
-@needs_reference
-def test_reference_archives_load_like_zipfile_and_json():
+@pytest.fixture(scope="module")
+def ref_data(reference_corpus):
+    "sourmash's test-data directory (shrunk; see the reference_corpus fixture)"
+    return os.path.join(reference_corpus, "tests", "test-data")
+
+
+def test_reference_archives_load_like_zipfile_and_json(ref_data):
     import json
-    paths = [p for p in glob.glob(os.path.join(REF_DATA, "**", "*.zip"), recursive=True)]
+    paths = [p for p in glob.glob(os.path.join(ref_data, "**", "*.zip"), recursive=True)]
     assert len(paths) > 10
     checked = 0
     for path in paths:
@@ -386,10 +388,9 @@ def test_reference_archives_load_like_zipfile_and_json():
     assert checked > 10
 
 
-@needs_reference
 @pytest.mark.parametrize("use_manifest", [True, False])
-def test_reference_all_zip_scenarios(use_manifest):                           # tests/test_index.py:821-927
-    path = os.path.join(REF_DATA, "prot", "all.zip")
+def test_reference_all_zip_scenarios(ref_data, use_manifest):                           # tests/test_index.py:821-927
+    path = os.path.join(ref_data, "prot", "all.zip")
     idx = ZipFileLinearIndex.load(path, use_manifest=use_manifest)
     assert len(list(idx.signatures())) == len(idx) == (8 if use_manifest else 7)
     all_idx = ZipFileLinearIndex.load(path, traverse_yield_all=True, use_manifest=use_manifest)
@@ -399,7 +400,7 @@ def test_reference_all_zip_scenarios(use_manifest):                           # 
     assert len(idx.select(moltype="DNA")) == (2 if use_manifest else 1)
     assert len(LinearIndex(idx.signatures()).select(moltype="DNA")) == (2 if use_manifest else 1)
     assert len(idx.select(ksize=19, moltype="protein")) == 2
-    abund = ZipFileLinearIndex.load(os.path.join(REF_DATA, "track_abund", "track_abund.zip"), use_manifest=use_manifest)
+    abund = ZipFileLinearIndex.load(os.path.join(ref_data, "track_abund", "track_abund.zip"), use_manifest=use_manifest)
     assert len(abund.select(abund=False)) == 2 and len(abund.select(abund=True)) == 2 and len(abund.select(abund=None)) == 2
     twice = ZipFileLinearIndex.load(path, use_manifest=use_manifest).select(ksize=19).select(moltype="protein")
     assert len(list(twice.signatures())) == 2

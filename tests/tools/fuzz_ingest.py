@@ -21,7 +21,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REFDATA = "/root/reference/tests/test-data"
+CORPUS = os.path.join(GOLDEN, "reference_corpus.tar.gz")         # sourmash's test data, shrunk
 
 CHILD = r'''
 import os, sys
@@ -78,15 +78,16 @@ def seeds():
             out.append(("sig", ".sig", fh.read()))
     with open(os.path.join(GOLDEN, "2.fa.sig"), "rb") as fh:
         out.append(("sig", ".sig.gz", gzip.compress(fh.read())))
-    zips = [p for p in sorted(glob.glob(os.path.join(REFDATA, "**", "*.zip"), recursive=True))
-            if "sbt" not in os.path.basename(p) and os.path.getsize(p) < 400_000]
-    for p in zips[:6]:
-        with open(p, "rb") as fh:
-            out.append(("zip", ".zip", fh.read()))
+    import tarfile
+    with tarfile.open(CORPUS) as tar:                               # sourmash's own collections (not the SBTs)
+        zips = [m for m in sorted(tar.getmembers(), key=lambda m: m.name)
+                if m.name.endswith(".zip") and "sbt" not in os.path.basename(m.name)]
+        for m in zips[:6]:
+            out.append(("zip", ".zip", tar.extractfile(m).read()))
     import io
     import zipfile
-    for method in (zipfile.ZIP_STORED, zipfile.ZIP_DEFLATED):       # collections made here (the only zip seeds where the
-        buf = io.BytesIO()                                          # reference checkout is absent): no manifest, two members
+    for method in (zipfile.ZIP_STORED, zipfile.ZIP_DEFLATED):       # collections made here (beside
+        buf = io.BytesIO()                                          # sourmash's): no manifest, two members
         with zipfile.ZipFile(buf, "w", method) as z:
             for name in ("2.fa.sig", "47.fa.sig"):
                 z.write(os.path.join(GOLDEN, name), "signatures/" + name)
